@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--config metric|inverted_pendulum|inv_double_pendulum|smgpr|swimmer|test_cascade]
-                    [--restarts R] [--through-api]
+                    [--restarts R] [--through-api] [--dump-outputs DIR]
 
 One bench "step" = one pass of the hot path over one batch: an H-step moment-matching rollout
 (policy moment match -> squash -> joint -> dynamics moment match -> glue -> reward, pilco.py:118-153)
@@ -15,6 +15,9 @@ H=40, RBF policy with 50 basis functions, fp64, synthetic seeded data, R=32 rest
 `--through-api` (any config) drives `PILCO.optimize_policy(restarts=R*N)` itself -- lock-step L-BFGS-B,
 taped forward + reverse sweep per evaluation, one all_gather of [loss | params] -- and reports wall-clock
 loss-evaluations x R x H / s.
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of each arm returned (trajectories, rewards,
+policy gradients; rank 0's restarts) as DIR/<name>.npy: the inputs are seeded, so two builds can be compared output
+for output.
 
 Rank 0 prints ONE JSON line.  `--impl reference` times the reference-equivalent CPU path
 (oracle/torch_port.py, all host threads it can use) on bounded samples of the same workload.
@@ -96,6 +99,24 @@ def make_policies(cfg, restart_ids, seed=0):
         Yc.append(0.1 * rng.randn(bf, U))
         lc.append(1.0 + 0.1 * rng.randn(U, Ds))
     return dict(Xc=np.stack(Xc), Yc=np.stack(Yc), lc=np.stack(lc))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, restart_ids, arrays):
+    """``--dump-outputs``: each array (leading dimension = restart) as ``<out_dir>/<name>.npy`` in float64, and the
+    global ids of the dumped restarts as ``restarts.npy``.  Above 64 MB in all, a fixed seeded sample of the
+    restarts is written instead, the same rows for every array."""
+    rows = np.arange(len(restart_ids))
+    row_bytes = 8 * sum(a[0].size for a in arrays.values())
+    if row_bytes * len(rows) > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // row_bytes)
+        rows = np.sort(np.random.RandomState(0).choice(len(rows), keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "restarts.npy"), np.asarray(restart_ids, dtype=np.float64)[rows])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64)[rows])
 
 
 def step_counts(cfg):
@@ -645,9 +666,8 @@ def run_ours(args, cfg):
     ms_e2e = timed(step_e2e, args.steps, args.warmup)
     ms_fb = ms_fb_e2e = ms_fbg = ms_fbg_e2e = None
     if split3 is not None:
-        kb = max(3, args.steps // 2)
-        ms_fb = timed(step_fwd_bwd, kb, 3)
-        ms_fb_e2e = timed(step_fwd_bwd_e2e, kb, 3)
+        ms_fb = timed(step_fwd_bwd, args.steps, 3)
+        ms_fb_e2e = timed(step_fwd_bwd_e2e, args.steps, 3)
         if G > 1:
             pipeline(3, False)
             ms_fbg = pipeline(args.steps, False) / args.steps
@@ -656,6 +676,17 @@ def run_ours(args, cfg):
     if sampler:
         sampler.stop_flag = True
         sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        out = {"rollout_traj_m": torch.cat([p.traj_m for p in split.plans]),
+               "rollout_traj_S": torch.cat([p.traj_S for p in split.plans]),
+               "rollout_reward": split.reward, "e2e_reward": h_out}
+        if split3 is not None:
+            fb_plans = [p for sp in gsplit3 for p in sp.plans] if G > 1 else split3.plans
+            out["fwd_bwd_reward"] = torch.cat([p.reward for p in fb_plans])
+            for k in gkeys:
+                out["fwd_bwd_grad_" + k] = torch.cat([p.gbuf[k] for p in fb_plans])
+            out["fwd_bwd_e2e_reward_grad"] = h_grad
+        dump_outputs(args.dump_outputs, my_ids, {k: v.cpu().numpy() for k, v in out.items()})
 
     total_steps = R * H * world
     value = total_steps / (ms_res * 1e-3)
@@ -861,7 +892,13 @@ def main():
     ap.add_argument("--stagger-ms", type=float, default=0.0, help="phase offset between the groups (default: one group's evaluation time / groups)")
     ap.add_argument("--through-api", action="store_true", help="drive PILCO.optimize_policy itself (lock-step L-BFGS-B, sharded restarts)")
     ap.add_argument("--maxiter", type=int, default=10, help="--through-api: L-BFGS-B iterations")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of each arm returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.through_api):
+        ap.error("--dump-outputs applies to the default arm (not --impl reference or --through-api)")
     cfg = CONFIGS[args.config]
     # Exactly ONE line on stdout (the JSON): everything any library writes to file descriptor 1 meanwhile (NCCL's
     # "NCCL version ..." banner is written by C code, not through sys.stdout) is sent to stderr; the JSON line is

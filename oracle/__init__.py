@@ -22,7 +22,7 @@ safe_port     numpy/torch transcription of the reference's safe_pilco_extension 
 fitc_staged   numpy statement of the FITC training objective with hand-derived adjoints (the algorithm a
               device SMGPR trainer implements), checked against torch autograd.
 mrun          a small MATLAB-subset interpreter that executes the reference's ``.m`` files
-              where they lie under /root/reference (this container only) to pin the
+              (the unmodified copies under ``tests/reference_tests/Matlab Code``) to pin the
               transcriptions and to generate ``tests/golden/*.npz``.
 
 Pinning status: the reference commits NO golden vectors (its tests call Octave live) and

@@ -3,10 +3,10 @@
 TEST INFRASTRUCTURE ONLY -- see ``oracle/__init__.py``.
 
 The reference's tests compare the Python code with ``tests/Matlab Code/*.m`` executed live in Octave
-(oct2py).  Octave is not installable here, so this module executes those ``.m`` files *where they lie*
-under ``/root/reference`` (nothing is copied): it is the "reference itself run here" that pins
-``oracle/matlab_port.py`` and generates ``tests/golden/*.npz`` (``tests/golden/make_golden.py``).
-It is only usable in the build container (``/root/reference`` does not exist on the GPU box).
+(oct2py).  Without Octave, this module executes those ``.m`` files -- by default the unmodified copies
+under ``tests/reference_tests/Matlab Code`` (checksums in ``tests/reference_tests/sha256sums.txt``): it is
+the "reference itself run here" that pins ``oracle/matlab_port.py`` and generates ``tests/golden/*.npz``
+(``tests/golden/make_golden.py``).
 
 Supported: function files with multiple outputs, nargin/nargout, if/elseif/else, for, return, persistent
 (ignored), struct field access/assignment, N-d indexing with ``end`` and ``:``, indexed assignment with
@@ -19,7 +19,7 @@ import re
 
 import numpy as np
 
-MDIR_DEFAULT = "/root/reference/tests/Matlab Code"
+MDIR_DEFAULT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "reference_tests", "Matlab Code")
 
 
 class MError(Exception):

@@ -1,10 +1,10 @@
 """Generate tests/golden/*.npz by EXECUTING the reference's MATLAB oracle files
-(/root/reference/tests/Matlab Code/*.m) with oracle/mrun.py, on the seeded recipes of the reference's tests
+(tests/reference_tests/Matlab Code/*.m) with oracle/mrun.py, on the seeded recipes of the reference's tests
 (tests/test_predictions.py, test_sparse_predictions.py, test_controllers.py, test_rewards.py,
 test_cascade.py) plus the BASELINE metric shape.  Hyper-parameters are fixed seeded values (the reference
 feeds whatever its optimisers return to the oracle; trajectories are not pinned, SURVEY.md section 4).
 
-Run in the build container only:   python tests/golden/make_golden.py
+    python tests/golden/make_golden.py
 """
 import os
 import sys

@@ -1,56 +1,39 @@
 """Drop-in check of the Python boundary (SURVEY.md section 8b-i): every class, method, property and module-level function
 the reference defines in pilco/ and safe_pilco_extension/ must exist here under the same import path with the same
-leading positional parameters.  Reads the reference's sources with ``ast`` (never imports or executes them), so it
-only runs where /root/reference is mounted (the build container); the GPU box skips it."""
-import ast
+leading positional parameters.  The reference's surface is stored in tests/golden/api_surface.json (read from its
+sources with ``ast`` by tests/golden/make_api_surface.py)."""
 import importlib
 import inspect
+import json
 import os
 
-import pytest
-
-REF = "/root/reference"
-MODULES = {
-    "pilco/models/mgpr.py": "pilco.models.mgpr",
-    "pilco/models/smgpr.py": "pilco.models.smgpr",
-    "pilco/models/pilco.py": "pilco.models.pilco",
-    "pilco/controllers.py": "pilco.controllers",
-    "pilco/rewards.py": "pilco.rewards",
-    "safe_pilco_extension/rewards_safe.py": "safe_pilco_extension.rewards_safe",
-    "safe_pilco_extension/safe_pilco.py": "safe_pilco_extension.safe_pilco",
-}
+SURFACE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "api_surface.json")
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pilco")), reason="reference tree not present")
 def test_public_surface_matches_reference():
     import pilco  # noqa: F401  (installs the alias modules)
     checked, problems = 0, []
-    for path, modname in MODULES.items():
-        tree = ast.parse(open(os.path.join(REF, path)).read())
+    for modname, ref in json.load(open(SURFACE)).items():
         mod = importlib.import_module(modname)
-        for node in tree.body:
-            if isinstance(node, ast.FunctionDef):
+        for name in ref["functions"]:
+            checked += 1
+            if not hasattr(mod, name):
+                problems.append("missing function %s.%s" % (modname, name))
+        for clsname, methods in ref["classes"].items():
+            cls = getattr(mod, clsname, None)
+            if cls is None:
+                problems.append("missing class %s.%s" % (modname, clsname))
+                continue
+            for name, ref_args in methods:
                 checked += 1
-                if not hasattr(mod, node.name):
-                    problems.append("missing function %s.%s" % (modname, node.name))
-            elif isinstance(node, ast.ClassDef):
-                cls = getattr(mod, node.name, None)
-                if cls is None:
-                    problems.append("missing class %s.%s" % (modname, node.name))
+                if not hasattr(cls, name):
+                    problems.append("missing %s.%s.%s" % (modname, clsname, name))
                     continue
-                for item in node.body:
-                    if not isinstance(item, ast.FunctionDef):
-                        continue
-                    checked += 1
-                    if not hasattr(cls, item.name):
-                        problems.append("missing %s.%s.%s" % (modname, node.name, item.name))
-                        continue
-                    static = inspect.getattr_static(cls, item.name)
-                    if isinstance(static, property):
-                        continue
-                    ref_args = [a.arg for a in item.args.args]
-                    our_args = list(inspect.signature(getattr(cls, item.name)).parameters)
-                    if our_args[:len(ref_args)] != ref_args:
-                        problems.append("signature %s.%s.%s: reference %s, here %s" % (modname, node.name, item.name, ref_args, our_args))
+                static = inspect.getattr_static(cls, name)
+                if isinstance(static, property):
+                    continue
+                our_args = list(inspect.signature(getattr(cls, name)).parameters)
+                if our_args[:len(ref_args)] != ref_args:
+                    problems.append("signature %s.%s.%s: reference %s, here %s" % (modname, clsname, name, ref_args, our_args))
     assert not problems, "\n".join(problems)
     assert checked >= 50

@@ -36,3 +36,27 @@ def test_reference_arm_prints_one_json_line():
     assert line["config"]["workload"] == bench.workload_string(cfg, cfg["R"])
     # every BASELINE.json config has a bench shape
     assert {"metric", "test_cascade", "inverted_pendulum", "inv_double_pendulum", "smgpr", "swimmer"} <= set(bench.CONFIGS)
+
+
+def test_dump_outputs_writes_float64_and_samples_above_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    ids = np.arange(10, 20)
+    arrays = {"traj": np.random.RandomState(1).rand(10, 3, 4), "reward": np.arange(10.0)}
+    bench.dump_outputs(str(tmp_path / "all"), ids, arrays)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "all" / (name + ".npy"))
+        assert got.dtype == np.float64 and np.array_equal(got, a)
+    assert np.array_equal(np.load(tmp_path / "all" / "restarts.npy"), ids)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8 * 13 * 4)            # room for 4 of the 10 restarts
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), ids, arrays)
+    rows = np.load(tmp_path / "s1" / "restarts.npy")
+    assert len(rows) == 4 and np.array_equal(rows, np.load(tmp_path / "s2" / "restarts.npy"))   # fixed sample
+    assert np.array_equal(np.load(tmp_path / "s1" / "reward.npy"), rows - 10)
+    assert np.array_equal(np.load(tmp_path / "s1" / "traj.npy"), arrays["traj"][(rows - 10).astype(int)])
+    assert sum(f.stat().st_size for f in (tmp_path / "s1").iterdir()) < 2 * 8 * 13 * 4 + 3 * 256   # + .npy headers
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--dump-outputs" in out.stderr

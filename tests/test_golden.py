@@ -70,13 +70,15 @@ def test_oracle_cascade_matches_reference_m_files():
     assert scaled_err(Mp[0], g["Mtraj"][:, -1]) < 1e-10 and scaled_err(Sp, g["Straj"][:, :, -1]) < 1e-9
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tests/Matlab Code"), reason="reference tree not present")
 def test_golden_regenerates_from_reference_sources():
-    """Re-execute two of the reference's .m files with oracle/mrun.py and compare with the committed vectors."""
+    """Re-execute two of the reference's .m files (the checksummed copies under tests/reference_tests) with
+    oracle/mrun.py and compare with the committed vectors."""
     from oracle import mrun
     g = load("gp0_a")
     M, S, V = mrun.run("gp0", dict(hyp=hyp_of(g["ell"], g["sf2"], g["sn2"]), inputs=g["X"], targets=g["Y"]), g["m"].T, g["s"], nout=3)
-    assert np.array_equal(M, g["M"]) and np.array_equal(S, g["S"]) and np.array_equal(V, g["V"])
+    # gp0.m goes through BLAS, whose summation order depends on the host's CPU kernel and thread count: over OpenBLAS
+    # core types x 1-8 threads the vectors reproduce to <= 1.4e-14 (M), 2.7e-12 (S, cancellation), 2.7e-14 (V)
+    assert scaled_err(M, g["M"]) < 1e-13 and scaled_err(S, g["S"]) < 1e-11 and scaled_err(V, g["V"]) < 1e-13
     g = load("gSin")
     M, S, C = mrun.run("gSin", g["m"].T, g["s"], float(g["e"]), nout=3)
     assert np.array_equal(M, g["M"]) and np.array_equal(S, g["S"])
