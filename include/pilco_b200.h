@@ -164,6 +164,23 @@ int pilco_fitc_factorize(int N, int Mi, int D, int E,
                          double* iK, int ldk, double* beta,
                          int* info, void* ws, size_t ws_bytes, pilco_stream_t stream);
 
+/* ---- prediction at deterministic inputs -------------------------------------------------------
+ * Replaces gpflow.models.GPR.predict_f / GPRFITC.predict_f, the methods users call on pilco.mgpr.models[i]
+ * (pilco/models/mgpr.py:28-36, smgpr.py:16-22; examples/"Hyperparameter setting and troubleshooting tips.ipynb",
+ * "Check the one-step predictions manually"), and through them predict_y / predict_log_density.  For B test points
+ * Xs and every output e, from the factors pilco_gp_factorize / pilco_fitc_factorize / pilco_gp_append leave (mode 0):
+ *   mean[b,e] = k*' beta_e,   var[b,e] = sf2_e - k*' iK_e k*   (latent, no noise),   k* = k_e(centres, Xs[b])
+ *   cov[e]    = K_e(Xs, Xs) - K*' iK_e K*                          (full_cov)
+ * Any of mean / var / cov may be NULL (not all three); var and cov need gp->iK.  The diagonal path is one fused kernel that
+ * never writes K* to memory and needs no workspace (pilco_gp_predict_workspace_bytes(..., 0) == 0); a point's result is
+ * bitwise independent of B and of its position in the batch.  cov needs 2 E B pad_n(n) doubles of workspace.
+ * gp must be unbatched (all *_bs == 0); one output i of an E-output model is predicted by passing E = 1 with ell, sf2,
+ * beta and iK offset to output i.  B == 0 is a no-op.  PILCO_ERR_UNSUPPORTED: n > 3472 centres. */
+size_t pilco_gp_predict_workspace_bytes(int n, int D, int E, int B, int full_cov);
+int    pilco_gp_predict(const pilco_gp_model* gp, int B, const double* Xs /*[B,D]*/,
+                        double* mean /*[B,E] or NULL*/, double* var /*[B,E] or NULL*/,
+                        double* cov /*[E,B,B] or NULL*/, void* ws, size_t ws_bytes, pilco_stream_t stream);
+
 /* ---- closed-form moments ---------------------------------------------------------------------
  * squash_sin (pilco/controllers.py:13-36; gSin.m:33-48), LinearController.compute_action
  * (controllers.py:46-58; conlin.m:50-62), ExponentialReward.compute_reward (rewards.py:19-51;

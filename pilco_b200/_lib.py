@@ -80,7 +80,9 @@ SIGNATURES = {
     "pilco_fitc_workspace_bytes": (C.c_size_t, [C.c_int] * 3),
     "pilco_fitc_factorize": (C.c_int, [C.c_int] * 4 + [c_dp] * 6 + [c_dp, C.c_int, c_dp, c_dp, c_dp,
                                                                   C.c_size_t, c_dp]),
-    "pilco_squash_sin": (C.c_int, [C.c_int, C.c_int] + [c_dp] * 7),
+    "pilco_gp_predict_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
+    "pilco_gp_predict": (C.c_int, [C.POINTER(GpModel), C.c_int] + [c_dp] * 5 + [C.c_size_t, c_dp]),
+    "pilco_squash_sin":(C.c_int, [C.c_int, C.c_int] + [c_dp] * 7),
     "pilco_linear_action": (C.c_int, [C.c_int] * 3 + [c_dp, c_ll, c_dp, c_ll] + [c_dp] * 6),
     "pilco_exp_reward": (C.c_int, [C.c_int, C.c_int] + [c_dp] * 8),
     "pilco_box_risk": (C.c_int, [C.c_int, C.c_int] + [c_dp] * 7),

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpilco_b200.so")
 SOURCES = ["abi.cu", "mm_forward.cu", "mm_backward.cu", "mm_tape.cu", "closed_forms.cu", "factorize.cu", "rollout.cu",
-           "rollout_bwd.cu", "microbench.cu"]
+           "rollout_bwd.cu", "microbench.cu", "gp_predict.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-rdc=false"]
 

@@ -1082,3 +1082,26 @@ int pilco_fitc_factorize(int N, int Mi, int D, int E, const double* X, const dou
 }
 
 }  // extern "C"
+
+// ---- full-covariance branch of pilco_gp_predict (gp_predict.cu) ----------------------------------------------------
+// GPR.predict_f / GPRFITC.predict_f with full_cov=True:  cov_e = K_e(Xs, Xs) - W K*',  W = K* iK_e,  K* = K_e(Xs, centres).
+// K* and W [E, B, pad64(n)] live in ws (the output is O(B^2) already); arguments validated by the caller.
+int gp_predict_full_cov(const pilco_gp_model* gp, int B, const double* Xs, double* cov, double* ws, cudaStream_t st) {
+    const int n = gp->n, D = gp->D, E = gp->E, ldn = pad64(n);
+    const long long ms = (long long)B * ldn, cs = (long long)B * B, ks = (long long)gp->ldk * gp->ldk;
+    double* Ks = ws;
+    double* W = Ks + (size_t)E * ms;
+    GramArgs gk{B, n, D, E, Xs, 0, gp->X, 0, gp->ell, 0, gp->sf2, 0, nullptr, 0, 0.0, Ks, ldn, ms, B, ldn, 0};
+    launch_pri(false, gram_kernel, dim3((ldn + 31) / 32, (B + 7) / 8, E), dim3(32, 8), 0, st, gk);
+    GramArgs gc{B, B, D, E, Xs, 0, Xs, 0, gp->ell, 0, gp->sf2, 0, nullptr, 0, 0.0, cov, B, cs, B, B, 0};
+    launch_pri(false, gram_kernel, dim3((B + 31) / 32, (B + 7) / 8, E), dim3(32, 8), 0, st, gc);
+    CUDA_LAUNCH_CHECK();
+    int rc = gemm(st, E, B, n, n, 0, 0, 1.0, Ks, ldn, ms, gp->iK, gp->ldk, ks, 0.0, W, ldn, ms);          // W = K* iK
+    if (rc) return rc;
+    rc = gemm(st, E, B, B, n, 0, 1, -1.0, W, ldn, ms, Ks, ldn, ms, 1.0, cov, B, cs);                        // cov -= W K*'
+    if (rc) return rc;
+    // W K*' is symmetric only up to round-off growing with cond(iK): average the two triangles (GPflow's K** - A'A is exact)
+    tri_op_kernel<<<dim3((B + 31) / 32, (B + 7) / 8, E), dim3(32, 8), 0, st>>>(B, cov, B, cs, 2);
+    CUDA_LAUNCH_CHECK();
+    return PILCO_OK;
+}

@@ -66,6 +66,14 @@ class DeviceGP:
         g.ldk = self.ldk
         return g
 
+    def output(self, i):
+        """Output ``i`` as a one-output model: same centres, views of row ``i`` of ell / sf2 / beta / iK (no copy)."""
+        if self.batched:
+            raise ValueError("DeviceGP.output: unbatched models only")
+        sl = slice(i, i + 1)
+        return DeviceGP(self.X, self.ell[sl], self.sf2[sl], self.beta[sl],
+                        self.iK[sl] if self.iK is not None else None, self.ldk, mode=self.mode)
+
 
 def gp_factorize(X, Y, ell, sf2, sn2, need_iK=True, mode=0):
     """pilco_gp_factorize.  Unbatched inputs ([n,D], [n,E], [E,D], [E], [E]) or batched with a leading B."""
@@ -215,6 +223,24 @@ def fitc_factorize(X, Z, Y, ell, sf2, sn2):
     gp = DeviceGP(Z, ell, sf2, beta, iK, ldk, mode=0)
     gp.info = info
     return gp
+
+
+def gp_predict(gp, Xs, full_cov=False, need_var=True):
+    """pilco_gp_predict: GP predictive at deterministic test points Xs [B,D] (GPR / GPRFITC.predict_f).
+    Returns mean [B,E] and var [B,E] (latent; None when not ``need_var``), or mean [B,E] and cov [E,B,B] with
+    ``full_cov``."""
+    Xs = dev(Xs).reshape(-1, gp.D)
+    B, E = Xs.shape[0], gp.E
+    d = device()
+    mean = torch.empty((B, E), dtype=F64, device=d)
+    var = torch.empty((B, E), dtype=F64, device=d) if need_var and not full_cov else None
+    cov = torch.empty((E, B, B), dtype=F64, device=d) if full_cov else None
+    wsb = lib.pilco_gp_predict_workspace_bytes(gp.n, gp.D, E, B, 1 if full_cov else 0)
+    ws = torch.empty(wsb // 8, dtype=F64, device=d) if wsb else None
+    g = gp.struct()
+    check(lib.pilco_gp_predict(C.byref(g), B, ptr(Xs), ptr(mean), ptr(var), ptr(cov), ptr(ws), wsb, stream_ptr()),
+          "gp_predict")
+    return (mean, cov) if full_cov else (mean, var)
 
 
 def mm_forward(gp, m, s):

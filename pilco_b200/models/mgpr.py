@@ -64,6 +64,28 @@ class GPRModel:
     def optimize(self, maxiter=None):
         return gp_training.minimize(self._loss, self.parameters, maxiter=maxiter)
 
+    # ---- gpflow prediction surface: routed through the owning MGPR / SMGPR (its resident device model, output i) -----
+    def _owner(self):
+        owner = getattr(self, "_mgpr", None)
+        if owner is None:
+            raise RuntimeError("GPRModel predictions run on the device model of the MGPR / SMGPR that created it")
+        return owner, self._output
+
+    def predict_f(self, Xnew, full_cov=False):
+        """gpflow GPR.predict_f: latent mean [B,1] and variance [B,1] (or covariance [1,B,B] with ``full_cov``)."""
+        owner, i = self._owner()
+        return owner._predict(Xnew, full_cov, output=i)
+
+    def predict_y(self, Xnew, full_cov=False):
+        """gpflow GPR.predict_y: predict_f plus the likelihood variance."""
+        owner, i = self._owner()
+        return owner._predict(Xnew, full_cov, output=i, noise=True)
+
+    def predict_log_density(self, data):
+        """gpflow GPR.predict_log_density: log N(y | mean, var + sn2) per point, [B]."""
+        owner, i = self._owner()
+        return owner._log_density(data, output=i)[:, 0]
+
 
 def randomize(model, mean=1, sigma=0.01):
     """pilco/models/mgpr.py:8-15"""
@@ -94,6 +116,12 @@ class MGPR:
             kern.lengthscales.prior = (1.1, 1.0 / 10.0)        # Gamma(alpha, rate)   mgpr.py:33
             kern.variance.prior = (1.5, 1.0 / 2.0)             # mgpr.py:34
             self.models.append(GPRModel((data[0], data[1][:, i:i + 1]), kern))
+        self._own_models()
+
+    def _own_models(self):
+        """Back-reference from each per-output model to this MGPR: its gpflow prediction methods run here."""
+        for i, model in enumerate(self.models):
+            model._mgpr, model._output = self, i
 
     def set_data(self, data):
         for i, model in enumerate(self.models):
@@ -265,3 +293,41 @@ class MGPR:
     def predict_on_noisy_inputs(self, m, s):
         """mgpr.py:77-79 -> (M [1,E], S [E,E], V [D,E])"""
         return self.predict_given_factorizations(m, s)
+
+    # ---- prediction at deterministic inputs (gpflow GPR / GPRFITC.predict_f of every output at once) -------------------
+    def _predict_device(self, Xnew, full_cov=False, output=None, noise=False):
+        """pilco_gp_predict on the resident device model (``device_gp``: same cache, refactorisation and incremental
+        append as the moment match).  CUDA tensors: mean [B,E'] and var [B,E'] or cov [E',B,B] (E' = 1 for ``output``)."""
+        if self.mm_mode != 0:
+            raise TypeError("%s is a deterministic GP (no predictive variance)" % type(self).__name__)
+        gp = self.device_gp()
+        sn2 = engine.dev(self.noise)
+        if output is not None:
+            gp, sn2 = gp.output(output), sn2[output:output + 1]
+        X = np.asarray(Xnew, dtype=np.float64).reshape(-1, gp.D)
+        mean, v = engine.gp_predict(gp, X, full_cov=full_cov)
+        if noise:
+            v = v + (torch.diag_embed(sn2[:, None].expand(-1, v.shape[-1])) if full_cov else sn2)
+        return mean, v
+
+    def _predict(self, Xnew, full_cov=False, output=None, noise=False):
+        mean, v = self._predict_device(Xnew, full_cov, output, noise)
+        return host(mean), host(v)
+
+    def _log_density(self, data, output=None):
+        mean, var = self._predict_device(data[0], output=output, noise=True)
+        Y = engine.dev(np.asarray(data[1], dtype=np.float64).reshape(mean.shape))
+        return host(-0.5 * (np.log(2.0 * np.pi) + torch.log(var) + (Y - mean) ** 2 / var))
+
+    def predict_f(self, Xnew, full_cov=False):
+        """Latent predictive of all E outputs at the points Xnew [B,D] (gpflow GPR.predict_f, or GPRFITC.predict_f under
+        SMGPR): mean [B,E] and var [B,E], or cov [E,B,B] with ``full_cov``.  One device call."""
+        return self._predict(Xnew, full_cov)
+
+    def predict_y(self, Xnew, full_cov=False):
+        """predict_f plus the likelihood variances ``noise`` (on the diagonal with ``full_cov``)."""
+        return self._predict(Xnew, full_cov, noise=True)
+
+    def predict_log_density(self, data):
+        """Gaussian log density of Y [B,E] under predict_y at X [B,D], data = (X, Y): [B,E]."""
+        return self._log_density(data)

@@ -1,6 +1,8 @@
 """SMGPR -- FITC sparse variant (drop-in for pilco/models/smgpr.py:11-52).  The FITC factorisation
 (smgpr.py:24-45, gp1.m:52-82) runs on the device (``pilco_fitc_factorize``); the moment match then runs
-over the M inducing points of output 0 (smgpr.py:47-52)."""
+over the M inducing points of output 0 (smgpr.py:47-52).  ``predict_f`` / ``predict_y`` / ``predict_log_density``
+(inherited from MGPR, and on every GPRFITCModel) use the same FITC factors, hence the inducing inputs of output 0 for
+every output: GPRFITC.predict_f of each output when the outputs share their inducing inputs."""
 import numpy as np
 import torch
 
@@ -43,6 +45,7 @@ class SMGPR(MGPR):
             kern = Kernel(data[0].shape[1])
             Z = np.random.rand(self.num_induced_points, self.num_dims)      # smgpr.py:20
             self.models.append(GPRFITCModel((data[0], data[1][:, i:i + 1]), kern, Z))
+        self._own_models()
 
     def optimize(self, restarts=1, maxiter=None):
         """FITC objective with trainable inducing inputs, on the device: all outputs and restarts in lock step, value
